@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- pgvector's distance hot path on B200, one JSON line per run (BASELINE.json metric and configs).
 
-  python bench.py [--config B] [--gpus N --steps K --warmup W] [--impl reference]
+  python bench.py [--config B] [--gpus N --steps K --warmup W] [--impl reference] [--dump-outputs DIR]
 
 --config selects the BASELINE.json configuration (default B = configs[1], the one the metric is quoted on):
 
@@ -81,7 +81,11 @@ def parse_args():
     ap.add_argument("--scan-impl", type=int, default=int(os.environ.get("VB_SCAN_IMPL", "2")),
                     help="0 = per-query LDG.128 scan, 1 = per-query cp.async.bulk (TMA) scan, 2 = library default "
                          "(query batches: tensor-core filter + exact re-score), 3 = list-major fp32, 4 = tensor-core filter")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="config B, product arm: write the ids and distances of the last timed step to DIR/*.npy")
     a = ap.parse_args()
+    if a.dump_outputs is not None and (a.config != "B" or a.impl != "ours"):
+        ap.error("--dump-outputs is implemented for config B, product arm")
     d = {"A": dict(rows=10_000, dim=128, lists=0, batch=1000, steps=100, warmup=3),
          "B": dict(rows=1_000_000, dim=1536, lists=1000, batch=2048, steps=100, warmup=3),
          "C": dict(rows=1_000_000, dim=768, lists=0, batch=10_000, steps=20, warmup=3),
@@ -290,6 +294,21 @@ def timed_steps(env, step, steps, warmup, extra_load=0):
     e1.record(env.stream)
     env.barrier()
     return env.max_over_ranks(e0.elapsed_time(e1))
+
+
+def dump_outputs(out_dir, arrays, budget=64 << 20):
+    """Write each array (rows = queries) as out_dir/<name>.npy in float32 / float64.  Above `budget` bytes in all, a
+    fixed seeded sample of the rows is written, with the sampled row numbers in row_index.npy."""
+    arrays = {name: np.asarray(a, dtype=np.float32 if a.dtype == np.float32 else np.float64) for name, a in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    per_row = sum(a[:1].nbytes for a in arrays.values()) + 8
+    if n * per_row > budget:
+        keep = np.sort(np.random.default_rng(0).choice(n, budget // per_row, replace=False))
+        arrays = {name: a[keep] for name, a in arrays.items()}
+        arrays["row_index"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------- config B: data, index (shared between the arms)
@@ -524,6 +543,7 @@ def measure_ivf(env, args, law, centers, offsets, grouped, order, full, queries)
     env.barrier()
     ms = env.max_over_ranks(e0.elapsed_time(e1))
     launches = pv.launch_count() - l0
+    last_step = (ids_dev.cpu().numpy(), dist_dev.cpu().numpy()) if args.dump_outputs is not None else None    # the last timed step's result
     prof = {name: pv.prof_read(p) for name, p in (("scan_items", pv.PROF_SCAN_ITEMS), ("scan_lists", pv.PROF_SCAN_LISTS),
                                                    ("topk", pv.PROF_TOPK), ("list_tc", pv.PROF_LIST_TC), ("centre_tc", pv.PROF_CENTRE_TC))}
     pv.prof_enable(False)
@@ -591,7 +611,7 @@ def measure_ivf(env, args, law, centers, offsets, grouped, order, full, queries)
     peak, _, peak_src = measured_peaks()
     roofline = roofline_ivf(args, ix, prof, traffic, cand_last, cand_all, B, ms, peak, peak_src, world)
     return dict(ix=ix, qps=qps, ms=ms, launches=int(launches), e2e=e2e, roofline=roofline, clocks=clocks, upload_s=upload_s,
-                cand_all=cand_all, qbatches=qbatches)
+                cand_all=cand_all, qbatches=qbatches, last_step=last_step)
 
 
 def roofline_ivf(args, ix, prof, traffic, cand_last, cand_all, B, ms, peak, peak_src, world):
@@ -828,6 +848,8 @@ def run_b_ours(args):
         torch.cuda.empty_cache()
     if env.rank == 0:
         m, ex = primary["m"], primary["extras"]
+        if args.dump_outputs is not None:
+            dump_outputs(args.dump_outputs, {"ids": m["last_step"][0], "distances": m["last_step"][1]})
         B = min(args.batch, args.queries)
         cfg = workload_b(args, primary["law"], primary["how"], dict(
             index_upload_s=m["upload_s"], candidates_per_query=m["cand_all"] / B,

@@ -12,13 +12,10 @@ import oracle as O
 from tests.harness import build as hbuild
 from tests.util import build_ivf_arrays, mixture
 
-HAVE_MOCK, _ = hbuild.build()
-pytestmark = pytest.mark.skipif(not HAVE_MOCK, reason="harness not built (needs the reference's headers)")
-
 
 @pytest.fixture(scope="module")
 def lib():
-    L = C.CDLL(hbuild.paths()[0])
+    L = C.CDLL(hbuild.build_broker())
     L.vb_ivf_create.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
     L.vb_ivf_load.argtypes = [C.c_void_p] * 5
     L.vb_ivf_free.argtypes = [C.c_void_p]

@@ -6,12 +6,13 @@ import subprocess
 
 import pytest
 
+from tests.harness.build import REF
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/src"
 EXT = os.path.join(ROOT, "pgvector_b200", "ext")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="pgvector source tree not present")
 @pytest.mark.parametrize("src", ["vb_ivfflat_scan.c", "vb_hnsw_scan.c", "vb_ivfflat_build.c", "vb_hnsw_build.c"])
 def test_glue_parses_against_reference_headers(src):
     cmd = ["gcc", "-fsyntax-only", "-std=gnu11", "-Wall", "-Werror", "-Wno-unused-function", "-Wno-comment",

@@ -1,13 +1,15 @@
 """CPU tests: the oracle against the reference's own known-answer outputs
 (tests/golden/distance_kat.json, transcribed from test/expected/*.out) and against
-the reference's halfutils.c/bitutils.c compiled verbatim (oracle/_ref)."""
+what the reference's halfutils.c/bitutils.c return on fixed inputs
+(tests/golden/ref_kernels.npz, recorded by tests/golden/make_ref_kernels.py)."""
 import math
+import os
 
 import numpy as np
 import pytest
 
 import oracle as O
-from tests.util import f32_to_half_bits, half_bits_to_f32, load_golden, parse_vector
+from tests.util import GOLDEN, f32_to_half_bits, half_bits_to_f32, load_golden, parse_vector
 
 ELEM = {"vector": O.VECTOR, "halfvec": O.HALFVEC, "bit": O.BIT}
 METRIC = {"l2_distance": O.L2, "inner_product": O.IP, "negative_inner_product": O.NEG_IP,
@@ -15,6 +17,7 @@ METRIC = {"l2_distance": O.L2, "inner_product": O.IP, "negative_inner_product": 
           "jaccard_distance": O.JACCARD}
 
 KAT = load_golden("distance_kat.json")["cases"]
+REF_KERNELS = np.load(os.path.join(GOLDEN, "ref_kernels.npz"))
 
 
 def _expect_float(text):
@@ -89,62 +92,49 @@ def test_half_conversion_matches_reference_and_numpy():
         (rng.standard_normal(500) * 1e-6).astype(np.float32),
     ])
     L = O.lib()
-    R = O.ref()
     npbits = f32_to_half_bits(xs)
     for x, nb in zip(xs, npbits):
         ob = L.pgv_float_to_half(float(x))
         assert ob == int(nb), (x, ob, nb)
-        if R is not None:
-            assert R.ref_float_to_half(float(x)) == ob, x
+    G = REF_KERNELS
+    for x, rb in zip(G["f2h_in"], G["f2h_out"]):
+        assert L.pgv_float_to_half(float(x)) == int(rb), x
     # widening: all 65536 patterns
     allh = np.arange(65536, dtype=np.uint16)
     npf = half_bits_to_f32(allh)
+    ref_h2f = dict(zip(G["h2f_in"].tolist(), G["h2f_out"].tolist()))
     for h in range(0, 65536, 7):
         f = L.pgv_half_to_float(h)
         if math.isnan(f):
             assert math.isnan(npf[h])
         else:
             assert f == npf[h]
-            if R is not None:
-                assert R.ref_half_to_float(h) == f
+            assert ref_h2f[h] == f
 
 
-@pytest.mark.skipif(O.ref() is None, reason="oracle/_ref not built (needs /root/reference)")
 def test_restated_half_and_bit_kernels_match_reference_build():
-    """The restatement vs the reference's own kernels on random inputs: bit kernels
+    """The restatement vs the reference's own kernels on stored random inputs: bit kernels
     exactly; half kernels within fp32 reassociation noise of the fp64 truth."""
-    R = O.ref()
-    rng = np.random.default_rng(1)
+    G = REF_KERNELS
     for dim in (1, 3, 8, 9, 64, 100, 768, 1537):
-        a = f32_to_half_bits(rng.standard_normal(dim))
-        b = f32_to_half_bits(rng.standard_normal(dim))
-        pa, pb = a.ctypes.data, b.ctypes.data
+        a, b = G[f"half_a_{dim}"], G[f"half_b_{dim}"]
+        ref_l2sq, ref_ip, ref_l1, ref_cos = G[f"half_out_{dim}"]
         truth = O.distance(O.HALFVEC, O.L2_SQUARED, a, b, f64=True)
-        for got in (R.ref_half_l2sq(dim, pa, pb), O.distance(O.HALFVEC, O.L2_SQUARED, a, b)):
+        for got in (ref_l2sq, O.distance(O.HALFVEC, O.L2_SQUARED, a, b)):
             assert abs(got - truth) <= 1e-5 * max(1.0, abs(truth))
         truth = O.distance(O.HALFVEC, O.IP, a, b, f64=True)
         scale = float(np.sum(np.abs(half_bits_to_f32(a) * half_bits_to_f32(b)))) + 1.0
-        for got in (R.ref_half_ip(dim, pa, pb), O.distance(O.HALFVEC, O.IP, a, b)):
+        for got in (ref_ip, O.distance(O.HALFVEC, O.IP, a, b)):
             assert abs(got - truth) <= 1e-5 * scale
         truth = O.distance(O.HALFVEC, O.L1, a, b, f64=True)
-        for got in (R.ref_half_l1(dim, pa, pb), O.distance(O.HALFVEC, O.L1, a, b)):
+        for got in (ref_l1, O.distance(O.HALFVEC, O.L1, a, b)):
             assert abs(got - truth) <= 1e-5 * max(1.0, truth)
-        cos_ref = 1.0 - min(1.0, max(-1.0, R.ref_half_cos(dim, pa, pb)))
+        cos_ref = 1.0 - min(1.0, max(-1.0, ref_cos))
         assert abs(cos_ref - O.distance(O.HALFVEC, O.COSINE, a, b)) <= 1e-5
     for nbits in (0, 1, 7, 8, 52, 63, 64, 65, 513, 1024, 4099):
-        nbytes = (nbits + 7) // 8
-        a = rng.integers(0, 256, size=max(nbytes, 1), dtype=np.uint8)[:nbytes].copy()
-        b = rng.integers(0, 256, size=max(nbytes, 1), dtype=np.uint8)[:nbytes].copy()
-        if nbits % 8 and nbytes:
-            mask = (0xFF << (8 - nbits % 8)) & 0xFF
-            a[-1] &= mask
-            b[-1] &= mask
-        a = np.ascontiguousarray(a)
-        b = np.ascontiguousarray(b)
-        pa = a.ctypes.data if nbytes else None
-        pb = b.ctypes.data if nbytes else None
-        assert R.ref_bit_hamming(nbytes, pa, pb) == O.distance(O.BIT, O.HAMMING, a, b, dim=nbits)
-        assert R.ref_bit_jaccard(nbytes, pa, pb) == O.distance(O.BIT, O.JACCARD, a, b, dim=nbits)
+        a, b = G[f"bit_a_{nbits}"], G[f"bit_b_{nbits}"]
+        assert int(G[f"bit_hamming_{nbits}"]) == O.distance(O.BIT, O.HAMMING, a, b, dim=nbits)
+        assert float(G[f"bit_jaccard_{nbits}"]) == O.distance(O.BIT, O.JACCARD, a, b, dim=nbits)
 
 
 def test_cross_type_equality_small_integers():
